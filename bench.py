@@ -14,6 +14,8 @@ A step = one pass of the hot path over one synthetic batch of `--rows` ChangeIte
 
 `--impl reference` times that CPU port instead (Go is not buildable here: no toolchain, deps not vendored).
 Launch: python bench.py --gpus N --steps K --warmup W   (N>1 under torch.distributed.run, one rank per GPU).
+`--dump-outputs DIR` writes what the last timed step computed on rank 0 to DIR/<name>.npy, so that two builds can be compared
+output for output (the inputs are seeded: the same arguments give the same batch).
 """
 from __future__ import annotations
 
@@ -21,6 +23,7 @@ import argparse
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
@@ -34,6 +37,12 @@ FALLBACK_HBM_GBS = 6650.0
 
 
 TRAFFIC_PROFILE = "profiles/r2h_traffic.json"   # written by scripts/ncu_summary.py from the capture under profiles/
+CACHE_DIR = tempfile.gettempdir()                  # generated inputs are cached here, never in the tree (which may be read-only)
+
+# --dump-outputs: bytes kept per output; each byte is stored as one float32, so 50 MB in all. Larger outputs are cut into
+# DUMP_CHUNK-byte chunks and a fixed seeded set of them is kept (the same chunks for the same output length).
+DUMP_BYTES = 6 << 20
+DUMP_CHUNK = 4096
 
 
 def bench_config(args, ncols: int) -> dict:
@@ -53,10 +62,10 @@ def load_peaks():
 
 
 def make_batch(rows: int, seed: int):
-    """Seeded synthetic batch; cached under /tmp so the two arms and every N reuse one generation."""
+    """Seeded synthetic batch; cached in the temporary directory so the two arms and every N reuse one generation."""
     from transferia_b200 import abi, workload
     schema = workload.hits_schema()
-    cache = f"/tmp/tfgpu_hits_{rows}_{seed}.npz"
+    cache = os.path.join(CACHE_DIR, f"tfgpu_hits_{rows}_{seed}.npz")
     if os.path.exists(cache):
         try:
             z = np.load(cache)
@@ -81,6 +90,47 @@ def make_batch(rows: int, seed: int):
     except Exception:
         pass
     return batch, schema
+
+
+def byte_sample(data: bytes, budget: int) -> np.ndarray:
+    """`data` as float32 byte values: all of it up to `budget` bytes, above that a seeded choice of whole DUMP_CHUNK-byte chunks."""
+    a = np.frombuffer(data, dtype=np.uint8)
+    if len(a) > budget:
+        pick = np.sort(np.random.default_rng(0).choice(len(a) // DUMP_CHUNK, budget // DUMP_CHUNK, replace=False))
+        a = a[(pick[:, None] * DUMP_CHUNK + np.arange(DUMP_CHUNK)).ravel()]
+    return a.astype(np.float32)
+
+
+def decode_frames(wire: bytes, raw_len: int):
+    """ClickHouse compressed frames ([16 checksum][0x82][u32 block size + 9][u32 raw size][LZ4 block]) decoded with stock liblz4:
+    (the bytes they carry, the number of frames). Raises on a frame that does not decode."""
+    import ctypes as C
+    import struct
+    lz = C.CDLL("liblz4.so.1")
+    out = C.create_string_buffer(max(1, raw_len)); pos = got = nf = 0
+    while pos < len(wire):
+        cs, rs = struct.unpack_from("<II", wire, pos + 17)
+        if wire[pos + 16] != 0x82 or got + rs > raw_len:
+            raise RuntimeError(f"frame {nf} at wire byte {pos}: bad header")
+        n = lz.LZ4_decompress_safe(wire[pos + 25: pos + 16 + cs], C.c_void_p(C.addressof(out) + got), cs - 9, rs)
+        if n != rs:
+            raise RuntimeError(f"frame {nf} at wire byte {pos}: liblz4 returned {n} of {rs} bytes")
+        pos += 16 + cs; got += rs; nf += 1
+    return out.raw[:got], nf
+
+
+def dump_outputs(eng, out_dir: str) -> None:
+    """What the last tfgpu_push_encode_resident call computed, as its caller fetches it: counts.npy (rows out, native block bytes,
+    frames, row errors; float64), raw_block.npy (the native block the frames compress) and wire_decoded.npy (the LZ4 frames decoded).
+    The compressed bytes themselves are not written: the match finder's hash-table inserts race, so which of several valid matches
+    a frame uses, and with it the compressed size, differs from run to run; what the frames decode to does not."""
+    st = eng.resident_stats()
+    raw = eng.resident_fetch(0, st["raw_bytes"])
+    decoded, n_frames = decode_frames(eng.resident_fetch(1, st["wire_bytes"]), st["raw_bytes"])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "counts.npy"), np.array([st["rows_out"], st["raw_bytes"], n_frames, st["n_errors"]], dtype=np.float64))
+    np.save(os.path.join(out_dir, "raw_block.npy"), byte_sample(raw, DUMP_BYTES))
+    np.save(os.path.join(out_dir, "wire_decoded.npy"), byte_sample(decoded, DUMP_BYTES))
 
 
 class ClockSampler(threading.Thread):
@@ -228,7 +278,7 @@ def extra_paths(eng, args):
     from transferia_b200 import abi, engine, workload
     sys.path.insert(0, ROOT)
     res = {}
-    cache = f"/tmp/tf_json_lines_{args.json_lines}.bin"
+    cache = os.path.join(CACHE_DIR, f"tf_json_lines_{args.json_lines}.bin")
     if os.path.exists(cache):
         text = open(cache, "rb").read(); fields = [dict(f) for f in workload.JSON_FIELDS]
     else:
@@ -279,7 +329,7 @@ def extra_paths(eng, args):
         res["debezium_emit_error"] = str(ex)
     # BASELINE configs[3]: Debezium CDC envelopes (12-field payload, schema-registry framed) -> parse -> filter_rows -> cast -> native block + LZ4
     try:
-        dcache = f"/tmp/tf_dbz_{args.dbz_msgs}.bin"
+        dcache = os.path.join(CACHE_DIR, f"tf_dbz_{args.dbz_msgs}.bin")
         if os.path.exists(dcache + ".npy"):
             ddata = open(dcache, "rb").read(); dends = np.load(dcache + ".npy"); dschema_text, dtable = workload.debezium_schema_text(), ("public", "events")
         else:
@@ -313,7 +363,7 @@ def extra_paths(eng, args):
         res["debezium_parse_error"] = str(ex)
     # BASELINE configs[4]: hits-shaped CSV -> parse -> cast -> ClickHouse native block (+ LZ4)
     try:
-        ccache = f"/tmp/tf_csv_{args.csv_rows}.bin"
+        ccache = os.path.join(CACHE_DIR, f"tf_csv_{args.csv_rows}.bin")
         cb, cschema = make_batch(args.csv_rows, workload.SEED)
         cschema = [dict(c, path=str(i)) for i, c in enumerate(cschema)]
         if os.path.exists(ccache):
@@ -433,7 +483,12 @@ def main():
     ap.add_argument("--e2e-mode", default="auto", choices=["auto", "one-phase", "two-phase"], help="end-to-end leg: tfgpu_push_encode (one-phase), tfgpu_push_encode_selective (two-phase), or both and report the faster (auto)")
     ap.add_argument("--gather-threads", type=int, default=0, help="host threads of the two-phase gather per pipeline (0: min(32, cores / pipelines / ranks))")
     ap.add_argument("--e2e-pipelines", type=int, default=4, help="host threads (one engine handle each) pushing batches concurrently in the end-to-end leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the device path; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
     if args.impl == "reference":
@@ -504,6 +559,8 @@ def main():
     ms_total = ev0.elapsed_time(ev1)
     for kk in eng.profile_read():        # events of the LAST timed step
         kernel_ms[kk["name"]] = kernel_ms.get(kk["name"], 0.0) + kk["ms"]
+    if args.dump_outputs and rank == 0:   # before any further call replaces the last timed step's outputs
+        dump_outputs(eng, args.dump_outputs)
     # average the dominant kernel over a few more (untimed) steps for a stable duration
     extra = 5
     acc = {}
