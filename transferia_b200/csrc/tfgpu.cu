@@ -129,6 +129,31 @@ int cuda_fail(tfgpu_engine* e, const CudaError& c) {
     return fail(e, c.e == cudaErrorMemoryAllocation ? TF_E_RETRY_OOM : TF_E_RETRY_LAUNCH, m);
 }
 
+// Body of an engine entry point: runs on the engine's device; what it throws becomes the call's return code and last_error
+// (FatalError derives from std::runtime_error, so it is caught first).
+template <class F> int guarded(tfgpu_engine* e, F&& body) {
+    try {
+        CK(cudaSetDevice(e->device));
+        return body();
+    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
+    catch (const CudaError& c) { return cuda_fail(e, c); }
+    catch (const std::bad_alloc&) { return fail(e, TF_E_RETRY_OOM, "host allocation failed"); }
+    catch (const std::exception& x) { return fail(e, TF_E_FATAL_CONFIG, x.what()); }
+}
+
+// Body of a host-only validator: `describe` builds the description, copied NUL-terminated into describe_out; what it throws
+// becomes the return code (a FatalError's own, else TF_E_FATAL_CONFIG) with its text in err_out.
+template <class F> int validated(char* describe_out, uint64_t cap, char* err_out, uint64_t err_cap, F&& describe) {
+    auto put = [](char* dst, uint64_t cap_, const std::string& s) { if (dst && cap_) { size_t n = s.size() < cap_ - 1 ? s.size() : cap_ - 1; std::memcpy(dst, s.data(), n); dst[n] = 0; } };
+    try {
+        const std::string d = describe();
+        if (describe_out && d.size() + 1 > cap) { put(err_out, err_cap, "describe buffer too small"); return TF_E_FATAL_ARG; }
+        put(describe_out, cap, d);
+        return TF_OK;
+    } catch (const tfplan::FatalError& f) { put(err_out, err_cap, f.what()); return f.code; }
+    catch (const std::exception& x) { put(err_out, err_cap, x.what()); return TF_E_FATAL_CONFIG; }
+}
+
 // encoding/json appendString with escapeHTML off, for column names (json.go:56-58)
 std::string host_json_quote_nohtml(const std::string& in) {
     static const char* hex = "0123456789abcdef";
@@ -161,6 +186,14 @@ int in_width(int tf) {
     case TF_INT64: case TF_UINT64: case TF_DOUBLE: case TF_INTERVAL: case TF_DATE: case TF_DATETIME: case TF_TIMESTAMP: return 8;
     }
     return 0;
+}
+
+// Kernel descriptor of column `c` read as `type`, without an output kind or a String / mask slot
+DCol plain_dcol(const tf_col& c, int type) {
+    DCol d; std::memset(&d, 0, sizeof d);
+    d.type = type; d.in_w = in_width(type); d.str_slot = -1; d.mask_slot = -1;
+    d.values = (const uint8_t*)c.values; d.validity = c.validity; d.offsets = c.offsets; d.heap = c.heap; d.aux = (const uint8_t*)c.aux;
+    return d;
 }
 
 template <typename T> T* carve(uint8_t*& p, size_t count) { T* r = (T*)p; p += align_up(count * sizeof(T), 256); return r; }
@@ -307,6 +340,52 @@ static void launch_offsets(tfgpu_engine* e, const uint32_t* d_len, uint64_t nrow
     e->prof_begin("k_offsets_sum", s); launch_k_offsets_sum(dim3(nchunks, nslots), 1024, 0, s, d_len, nrows, nchunks, cs); e->prof_end(s);
     e->prof_begin("k_offsets_chunks", s); launch_k_offsets_chunks(nslots, 32, 0, s, cs, nchunks, d_tot); e->prof_end(s);
     e->prof_begin("k_offsets_write", s); launch_k_offsets_write(dim3(nchunks, nslots), 1024, 0, s, d_len, nrows, nchunks, cs, d_tot, d_off); e->prof_end(s);
+}
+
+// The device parsers (CSV, JSON lines, Debezium) type their input in two passes: pass one writes the fixed-width values and the
+// byte length of every text cell, pass two copies the text cells into per-column heaps placed from those lengths. What lies between
+// and after the passes is shared; the pass kernels and their arguments stay per parser.
+
+// Layout of a staging arena: every region starts at a multiple of 256 bytes (an empty one still takes 256).
+struct ArenaLayout {
+    size_t total = 0;
+    size_t operator()(size_t bytes) { const size_t at = total; total += align_up(bytes ? bytes : 1, 256); return at; }
+};
+
+// Text heaps of the var-width columns (slots) of a parsed batch
+struct VarHeaps {
+    std::vector<uint64_t> total, base; uint8_t* heap = nullptr;
+    explicit VarHeaps(int nslots) : total(nslots ? nslots : 1, 0), base(nslots ? nslots : 1, 0) {}
+};
+
+// Between the passes: scans the cell lengths d_len [nslots][nrows] into offsets d_off [nslots][nrows + 1], reads the slot totals
+// back (one synchronise), gives every slot a 16-byte-aligned base in in_arena and uploads the bases to d_base for pass two.
+// in_arena is free during a parse: the parsed batch is device resident, so stage_input does not run.
+void place_heaps(tfgpu_engine* e, VarHeaps& h, const uint32_t* d_len, uint64_t nrows, int nslots, uint32_t* d_off, uint64_t* d_tot, uint64_t* d_base, const char* what) {
+    cudaStream_t s = e->stream;
+    launch_offsets(e, d_len, nrows, (uint32_t)nslots, d_off, d_tot, s);
+    CK(cudaMemcpyAsync(h.total.data(), d_tot, (size_t)nslots * 8, cudaMemcpyDeviceToHost, s)); CK(cudaStreamSynchronize(s));
+    uint64_t run = 0; for (int k = 0; k < nslots; k++) { h.base[k] = run; run += align_up(h.total[k], 16); }
+    if (run >= (1ull << 32)) throw tfplan::FatalError(TF_E_FATAL_ARG, std::string(what) + ": a text column exceeds 4 GiB");
+    e->in_arena.ensure(run + 256); h.heap = e->in_arena.p;
+    CK(cudaMemcpyAsync(d_base, h.base.data(), (size_t)nslots * 8, cudaMemcpyHostToDevice, s));
+}
+
+// what pass one writes beside the values: validity bitmaps (JSON, Debezium), nanoseconds of time columns and tags of `any` columns (CSV, JSON)
+void parsed_extras(const CsvColDev& h, tf_col& d) { d.aux = h.w ? (const void*)h.aux32 : h.aux8; }
+void parsed_extras(const JsnColDev& h, tf_col& d) { d.aux = h.w ? (const void*)h.aux32 : h.aux8; d.validity = (const uint8_t*)h.validity; }
+void parsed_extras(const DbzColDev& h, tf_col& d) { d.validity = (const uint8_t*)h.validity; }
+
+// The parsed columns as the device-resident batch the chain reads (`dev` holds its columns); a text column takes its slot's
+// offsets (d_off) and heap.
+template <class ColDev> tf_batch parsed_batch(const std::vector<ColDev>& hc, uint64_t nrows, const uint32_t* d_off, const VarHeaps& h, std::vector<tf_col>& dev) {
+    dev.assign(hc.size(), tf_col{});
+    for (size_t c = 0; c < hc.size(); c++) {
+        tf_col& d = dev[c]; d.type = hc[c].tf; parsed_extras(hc[c], d);
+        if (hc[c].w) d.values = hc[c].values;
+        else { const int k = hc[c].slot; d.offsets = d_off + (size_t)k * (nrows + 1); d.heap = h.heap ? h.heap + h.base[k] : nullptr; d.heap_len = h.total[k]; }
+    }
+    return tf_batch{nrows, (uint32_t)hc.size(), TF_MEM_DEVICE, dev.data(), nullptr};
 }
 
 // Launch the whole fused chain on e->stream. `cols_host` holds DEVICE pointers.
@@ -548,6 +627,29 @@ void run_chain(tfgpu_engine* e, PlanDev& pd, const tf_batch* in, const tf_col* d
 static bool wire_is_ser(int wire_fmt) { const int b = wire_fmt & 0xff; return (b == TF_WIRE_SER_JSON || b == TF_WIRE_SER_CSV) && (wire_fmt & ~(0xff | TF_WIRE_F_CLOSING_NEWLINE | TF_WIRE_F_ANY_AS_STRING)) == 0; }
 static bool wire_known(int wire_fmt) { return wire_fmt == TF_WIRE_CH_NATIVE || wire_fmt == TF_WIRE_CH_NATIVE_LZ4 || wire_fmt == TF_WIRE_CH_JSONEACHROW || wire_is_ser(wire_fmt); }
 
+// The plan `plan_id` names, or nullptr for a missing engine or an id out of range (the call answers TF_E_FATAL_ARG).
+static PlanDev* plan_arg(tfgpu_engine* e, int plan_id) { return (e && plan_id >= 0 && plan_id < (int)e->plans.size()) ? e->plans[plan_id].get() : nullptr; }
+// A wire format the encoder writes, with a sink in the plan unless it is a serializer format; columnar_ok: the parsers' 0 (rows columnar).
+static void check_wire(const PlanDev& pd, int wire_fmt, bool columnar_ok) {
+    if (columnar_ok && wire_fmt == 0) return;
+    if (!wire_known(wire_fmt)) throw tfplan::FatalError(TF_E_FATAL_UNSUPPORTED, "wire format not implemented");
+    if (!wire_is_ser(wire_fmt) && !pd.plan.has_sink) throw tfplan::FatalError(TF_E_FATAL_CONFIG, "plan was built without a sink");
+}
+static void check_batch(const PlanDev& pd, const tf_batch* in) {
+    if (in->ncols != pd.plan.in_schema.size()) throw tfplan::FatalError(TF_E_FATAL_ARG, "batch column count does not match the plan schema");
+    if (in->nrows >= (1ull << 31)) throw tfplan::FatalError(TF_E_FATAL_ARG, "batch too large (>= 2^31 rows)");
+}
+// Message end offsets of a parser call (end_of(m) = end of message m): non-decreasing, inside the buffer, the last one at its end.
+template <class End> static void check_msg_ends(uint64_t len, uint32_t n_msgs, End end_of) {
+    uint64_t prev = 0;
+    for (uint32_t m = 0; m < n_msgs; m++) {
+        const uint64_t end = end_of(m);
+        if (end < prev || end > len) throw tfplan::FatalError(TF_E_FATAL_ARG, "message ends must be non-decreasing and inside the buffer");
+        prev = end;
+    }
+    if (prev != len) throw tfplan::FatalError(TF_E_FATAL_ARG, "the messages must cover the whole buffer");
+}
+
 extern "C" {
 
 const char* tfgpu_version(void) { return "tfgpu 0.1.0 sm_100a"; }
@@ -641,17 +743,14 @@ int tfgpu_engine_set_stream(tfgpu_engine* e, void* cuda_stream) {
 int tfgpu_plan(tfgpu_engine* e, const char* ns, const char* name, const char* schema_json, const char* transformers_json,
                const char* sink_json, int* plan_id) {
     if (!e || !schema_json || !plan_id || !name) return TF_E_FATAL_ARG;
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
         auto pd = std::make_unique<PlanDev>();
         pd->plan = tfplan::build_plan(ns ? ns : "", name, schema_json, transformers_json ? transformers_json : "", sink_json ? sink_json : "");
         upload_plan(e, *pd);
         e->plans.push_back(std::move(pd));
         *plan_id = (int)e->plans.size() - 1;
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
-    catch (const std::exception& x) { return fail(e, TF_E_FATAL_CONFIG, x.what()); }
+    });
 }
 
 // Host-only: build the plan (Suitable / ResultSchema chain, filter grammar, ClickHouse types) without touching a
@@ -659,15 +758,10 @@ int tfgpu_plan(tfgpu_engine* e, const char* ns, const char* name, const char* sc
 // reference's transformers: cmd/trcli/config/model.go:57-72).
 int tfgpu_plan_validate(const char* ns, const char* name, const char* schema_json, const char* transformers_json,
                         const char* sink_json, char* describe_out, uint64_t cap, char* err_out, uint64_t err_cap) {
-    auto put = [](char* dst, uint64_t cap_, const std::string& s) { if (dst && cap_) { size_t n = s.size() < cap_ - 1 ? s.size() : cap_ - 1; std::memcpy(dst, s.data(), n); dst[n] = 0; } };
     if (!schema_json || !name) return TF_E_FATAL_ARG;
-    try {
-        tfplan::Plan pl = tfplan::build_plan(ns ? ns : "", name, schema_json, transformers_json ? transformers_json : "", sink_json ? sink_json : "");
-        if (describe_out && pl.describe.size() + 1 > cap) { put(err_out, err_cap, "describe buffer too small"); return TF_E_FATAL_ARG; }
-        put(describe_out, cap, pl.describe);
-        return TF_OK;
-    } catch (const tfplan::FatalError& f) { put(err_out, err_cap, f.what()); return f.code; }
-    catch (const std::exception& x) { put(err_out, err_cap, x.what()); return TF_E_FATAL_CONFIG; }
+    return validated(describe_out, cap, err_out, err_cap, [&] {
+        return tfplan::build_plan(ns ? ns : "", name, schema_json, transformers_json ? transformers_json : "", sink_json ? sink_json : "").describe;
+    });
 }
 
 const char* tfgpu_plan_describe(tfgpu_engine* e, int plan_id) {
@@ -677,39 +771,34 @@ const char* tfgpu_plan_describe(tfgpu_engine* e, int plan_id) {
 
 static const uint8_t* stage_input(tfgpu_engine* e, const tf_batch* in, std::vector<tf_col>& dev, DevBuf* arena_opt = nullptr);
 int tfgpu_push_encode_resident(tfgpu_engine* e, int plan_id, int wire_fmt, const tf_batch* in) {
-    if (!e || !in || plan_id < 0 || plan_id >= (int)e->plans.size()) return TF_E_FATAL_ARG;
-    PlanDev& pd = *e->plans[plan_id];
-    if (!pd.plan.has_sink) return fail(e, TF_E_FATAL_CONFIG, "plan was built without a sink");
-    if (in->mem != TF_MEM_DEVICE) return fail(e, TF_E_FATAL_ARG, "tfgpu_push_encode_resident needs a TF_MEM_DEVICE batch");
-    if (in->ncols != pd.plan.in_schema.size()) return fail(e, TF_E_FATAL_ARG, "batch column count does not match the plan schema");
-    if (wire_fmt != TF_WIRE_CH_NATIVE && wire_fmt != TF_WIRE_CH_NATIVE_LZ4) return fail(e, TF_E_FATAL_UNSUPPORTED, "wire format not implemented");
-    if (in->nrows >= (1ull << 31)) return fail(e, TF_E_FATAL_ARG, "batch too large (>= 2^31 rows)");
-    try {
-        CK(cudaSetDevice(e->device));
+    PlanDev* pd = plan_arg(e, plan_id);
+    if (!pd || !in) return TF_E_FATAL_ARG;
+    return guarded(e, [&] {
+        if (!pd->plan.has_sink) return fail(e, TF_E_FATAL_CONFIG, "plan was built without a sink");
+        if (in->mem != TF_MEM_DEVICE) return fail(e, TF_E_FATAL_ARG, "tfgpu_push_encode_resident needs a TF_MEM_DEVICE batch");
+        check_batch(*pd, in);
+        if (wire_fmt != TF_WIRE_CH_NATIVE && wire_fmt != TF_WIRE_CH_NATIVE_LZ4) return fail(e, TF_E_FATAL_UNSUPPORTED, "wire format not implemented");
         std::vector<tf_col> dev; const uint8_t* dev_kinds = stage_input(e, in, dev);    // device pointers pass through; TF_COL_LENS8 / 16 lengths become offsets
-        run_chain(e, pd, in, dev.data(), dev_kinds, wire_fmt);
+        run_chain(e, *pd, in, dev.data(), dev_kinds, wire_fmt);
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
+    });
 }
 
 int tfgpu_resident_stats(tfgpu_engine* e, uint64_t* rows_out, uint64_t* raw_bytes, uint64_t* wire_bytes, uint64_t* n_errors) {
     if (!e) return TF_E_FATAL_ARG;
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
         join_tail(e);
         DState st; CK(cudaMemcpyAsync(&st, e->d_state, sizeof st, cudaMemcpyDeviceToHost, e->stream)); CK(cudaStreamSynchronize(e->stream));
         if (rows_out) *rows_out = st.n_kept; if (raw_bytes) *raw_bytes = st.raw_total;
         if (wire_bytes) *wire_bytes = e->last_wire_fmt == TF_WIRE_CH_NATIVE_LZ4 ? st.wire_total : st.raw_total;
         if (n_errors) *n_errors = st.n_errors;
         return TF_OK;
-    } catch (const CudaError& c) { return cuda_fail(e, c); }
+    });
 }
 
 int tfgpu_resident_fetch(tfgpu_engine* e, int what, uint8_t* dst, uint64_t cap) {
     if (!e || !dst) return TF_E_FATAL_ARG;
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
         join_tail(e);
         DState st; CK(cudaMemcpyAsync(&st, e->d_state, sizeof st, cudaMemcpyDeviceToHost, e->stream)); CK(cudaStreamSynchronize(e->stream));
         const bool wire = what == 1 && e->last_wire_fmt == TF_WIRE_CH_NATIVE_LZ4;
@@ -717,50 +806,41 @@ int tfgpu_resident_fetch(tfgpu_engine* e, int what, uint8_t* dst, uint64_t cap) 
         if (n > cap) return fail(e, TF_E_FATAL_ARG, "destination too small");
         CK(cudaMemcpyAsync(dst, wire ? e->wire.p : e->raw.p, n, cudaMemcpyDeviceToHost, e->stream)); CK(cudaStreamSynchronize(e->stream));
         return TF_OK;
-    } catch (const CudaError& c) { return cuda_fail(e, c); }
+    });
 }
 
-static void fetch_errors(tfgpu_engine* e, uint64_t n, tfgpu_result* r);
 static void finish_wire(tfgpu_engine* e, uint64_t n, int wire_fmt, tfgpu_result* r);
 
 int tfgpu_push_encode(tfgpu_engine* e, int plan_id, int wire_fmt, const tf_batch* in, tfgpu_result** out) {
-    if (!e || !in || !out || plan_id < 0 || plan_id >= (int)e->plans.size()) return TF_E_FATAL_ARG;
+    PlanDev* pd = plan_arg(e, plan_id);
+    if (!pd || !in || !out) return TF_E_FATAL_ARG;
     *out = nullptr;
-    PlanDev& pd = *e->plans[plan_id];
-    if (!wire_known(wire_fmt)) return fail(e, TF_E_FATAL_UNSUPPORTED, "wire format not implemented");
-    if (!wire_is_ser(wire_fmt) && !pd.plan.has_sink) return fail(e, TF_E_FATAL_CONFIG, "plan was built without a sink");
-    if (in->ncols != pd.plan.in_schema.size()) return fail(e, TF_E_FATAL_ARG, "batch column count does not match the plan schema");
-    if (in->nrows >= (1ull << 31)) return fail(e, TF_E_FATAL_ARG, "batch too large (>= 2^31 rows)");
-    try {
-        CK(cudaSetDevice(e->device));
-        const uint64_t n = in->nrows;
+    return guarded(e, [&] {
+        check_wire(*pd, wire_fmt, false);
+        check_batch(*pd, in);
         std::vector<tf_col> dev; const uint8_t* dev_kinds = stage_input(e, in, dev);
-        cudaStream_t s = e->stream;
-        run_chain(e, pd, in, dev.data(), dev_kinds, wire_fmt);
+        run_chain(e, *pd, in, dev.data(), dev_kinds, wire_fmt);
         auto r = std::make_unique<tfgpu_result>();
-        finish_wire(e, n, wire_fmt, r.get());
+        finish_wire(e, in->nrows, wire_fmt, r.get());
         *out = r.release();
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
-    catch (const std::bad_alloc&) { return fail(e, TF_E_RETRY_OOM, "host allocation failed"); }
+    });
 }
 
 // Two-phase push: only the predicate columns cross PCIe first; k_filter answers with the keep flags; the host gathers the kept rows
 // (tfgpu_batch_gather, multi-threaded) and only those go through the whole chain. Same result as tfgpu_push_encode: every transformer is
 // row-local, filters keep the rows they kept before, and the rows phase one dropped with an error are reported from phase one.
 int tfgpu_push_encode_selective(tfgpu_engine* e, int plan_id, int wire_fmt, const tf_batch* in, int threads, tfgpu_result** out) {
-    if (!e || !in || !out || plan_id < 0 || plan_id >= (int)e->plans.size()) return TF_E_FATAL_ARG;
-    PlanDev& pd = *e->plans[plan_id];
-    const tfplan::Plan& pl = pd.plan;
+    PlanDev* pd = plan_arg(e, plan_id);
+    if (!pd || !in || !out) return TF_E_FATAL_ARG;
+    const tfplan::Plan& pl = pd->plan;
     const uint64_t n = in->nrows; const size_t nc = pl.in_schema.size();
-    if (in->mem != TF_MEM_HOST || in->ncols != nc || pd.n_fsteps == 0 || n < 8192 || !wire_known(wire_fmt)) return tfgpu_push_encode(e, plan_id, wire_fmt, in, out);
+    if (in->mem != TF_MEM_HOST || in->ncols != nc || pd->n_fsteps == 0 || n < 8192 || !wire_known(wire_fmt)) return tfgpu_push_encode(e, plan_id, wire_fmt, in, out);
     std::vector<uint8_t> pred(nc, 0);
     for (const auto& fs : pl.filters) for (const auto& ex : fs.exprs) for (const auto& t : ex) if (t.col >= 0 && (size_t)t.col < nc) pred[t.col] = 1;
     for (size_t c = 0; c < nc; c++) if (pred[c] && in->cols[c].type != pl.in_schema[c].tf) return tfgpu_push_encode(e, plan_id, wire_fmt, in, out);   // loose predicate column: Strictify first, one phase
     *out = nullptr;
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
         join_tail(e);
         cudaStream_t s = e->stream;
         static const bool trace = std::getenv("TFGPU_SELECTIVE_TRACE") != nullptr;
@@ -771,11 +851,7 @@ int tfgpu_push_encode_selective(tfgpu_engine* e, int plan_id, int wire_fmt, cons
         const tf_batch b1{n, (uint32_t)nc, TF_MEM_HOST, pc.data(), in->kinds};
         std::vector<tf_col> dev; const uint8_t* dev_kinds = stage_input(e, &b1, dev);
         std::vector<DCol> hc(nc);
-        for (size_t c = 0; c < nc; c++) {
-            DCol& d = hc[c]; std::memset(&d, 0, sizeof d);
-            d.type = pl.in_schema[c].tf; d.in_w = in_width(d.type); d.str_slot = -1; d.mask_slot = -1;
-            d.values = (const uint8_t*)dev[c].values; d.validity = dev[c].validity; d.offsets = dev[c].offsets; d.heap = dev[c].heap; d.aux = (const uint8_t*)dev[c].aux;
-        }
+        for (size_t c = 0; c < nc; c++) hc[c] = plain_dcol(dev[c], pl.in_schema[c].tf);
         if (e->d_cols_cap < nc) { if (e->d_cols) CK(cudaFree(e->d_cols)); CK(cudaMalloc(&e->d_cols, sizeof(DCol) * nc)); e->d_cols_cap = nc; }
         CK(cudaMemcpyAsync(e->d_cols, hc.data(), sizeof(DCol) * nc, cudaMemcpyHostToDevice, s));
         CK(cudaMemsetAsync(e->d_state, 0, sizeof(DState), s));
@@ -783,7 +859,7 @@ int tfgpu_push_encode_selective(tfgpu_engine* e, int plan_id, int wire_fmt, cons
         const size_t flags_bytes = align_up(3 * n, 256);
         e->sel_stage.ensure(flags_bytes + (size_t)nb * 4 + 256);
         uint8_t* B = e->sel_stage.p;
-        FilterArgs fa{e->d_cols, dev_kinds, n, pd.d_fsteps, pd.n_fsteps, pd.d_expr_off, pd.d_terms, pd.d_blob, B, B + n, B + 2 * n, (uint32_t*)(B + flags_bytes), e->d_state, nullptr, nullptr, 0};
+        FilterArgs fa{e->d_cols, dev_kinds, n, pd->d_fsteps, pd->n_fsteps, pd->d_expr_off, pd->d_terms, pd->d_blob, B, B + n, B + 2 * n, (uint32_t*)(B + flags_bytes), e->d_state, nullptr, nullptr, 0};
         e->prof_n = 0;
         e->prof_begin("k_filter", s); launch_k_filter(nb, 256, 0, s, fa); e->prof_end(s);
         if (e->sel_host_cap < 3 * n) { if (e->sel_host) CK(cudaFreeHost(e->sel_host)); e->sel_host = nullptr; e->sel_host_cap = 0; const size_t want = align_up(3 * n + 3 * n / 4 + 4096, 1 << 16); CK(cudaMallocHost(&e->sel_host, want)); e->sel_host_cap = want; }
@@ -799,7 +875,7 @@ int tfgpu_push_encode_selective(tfgpu_engine* e, int plan_id, int wire_fmt, cons
         const auto t_2 = std::chrono::steady_clock::now();
         // ---- phase two: the whole chain over the kept rows
         std::vector<tf_col> dev2; const uint8_t* dev_kinds2 = stage_input(e, kept, dev2);
-        run_chain(e, pd, kept, dev2.data(), dev_kinds2, wire_fmt);
+        run_chain(e, *pd, kept, dev2.data(), dev_kinds2, wire_fmt);
         auto r = std::make_unique<tfgpu_result>();
         finish_wire(e, kept->nrows, wire_fmt, r.get());
         r->rows_in = n;
@@ -818,9 +894,7 @@ int tfgpu_push_encode_selective(tfgpu_engine* e, int plan_id, int wire_fmt, cons
         }
         *out = r.release();
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
-    catch (const std::bad_alloc&) { return fail(e, TF_E_RETRY_OOM, "host allocation failed"); }
+    });
 }
 uint64_t tfgpu_engine_h2d_bytes(const tfgpu_engine* e) { return e ? e->h2d_bytes : 0; }
 
@@ -980,24 +1054,28 @@ static void finish_wire(tfgpu_engine* e, uint64_t n, int wire_fmt, tfgpu_result*
     CK(cudaStreamSynchronize(s));
 }
 
+// The plan's chain over a parser's device-resident batch: the rows come back columnar (wire_fmt 0) or as wire bytes.
+static std::unique_ptr<tfgpu_result> chain_parsed(tfgpu_engine* e, PlanDev& pd, const tf_batch& staged, const uint8_t* kinds, const uint8_t* pre_err, int wire_fmt) {
+    run_chain(e, pd, &staged, staged.cols, kinds, wire_fmt == 0 ? TF_WIRE_COLUMNAR_INTERNAL : wire_fmt, pre_err);
+    auto r = std::make_unique<tfgpu_result>();
+    if (wire_fmt == 0) finish_columnar(e, pd, staged.nrows, r.get()); else finish_wire(e, staged.nrows, wire_fmt, r.get());
+    return r;
+}
+
 // TransformerResult{Transformed, Errors}: the kept rows come back columnar in host memory owned by the result.
 int tfgpu_push_columns(tfgpu_engine* e, int plan_id, const tf_batch* in, tfgpu_result** out) {
-    if (!e || !in || !out || plan_id < 0 || plan_id >= (int)e->plans.size()) return TF_E_FATAL_ARG;
+    PlanDev* pd = plan_arg(e, plan_id);
+    if (!pd || !in || !out) return TF_E_FATAL_ARG;
     *out = nullptr;
-    PlanDev& pd = *e->plans[plan_id];
-    if (in->ncols != pd.plan.in_schema.size()) return fail(e, TF_E_FATAL_ARG, "batch column count does not match the plan schema");
-    if (in->nrows >= (1ull << 31)) return fail(e, TF_E_FATAL_ARG, "batch too large (>= 2^31 rows)");
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
+        check_batch(*pd, in);
         std::vector<tf_col> dev; const uint8_t* dev_kinds = stage_input(e, in, dev);
-        run_chain(e, pd, in, dev.data(), dev_kinds, TF_WIRE_COLUMNAR_INTERNAL);
+        run_chain(e, *pd, in, dev.data(), dev_kinds, TF_WIRE_COLUMNAR_INTERNAL);
         auto r = std::make_unique<tfgpu_result>();
-        finish_columnar(e, pd, in->nrows, r.get());
+        finish_columnar(e, *pd, in->nrows, r.get());
         *out = r.release();
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
-    catch (const std::bad_alloc&) { return fail(e, TF_E_RETRY_OOM, "host allocation failed"); }
+    });
 }
 
 // Queue Debezium serializer for columns without a database-specific original_type (Emitter.EmitKV
@@ -1110,9 +1188,8 @@ void dbz_build_template(PlanDev& pd, const std::string& opts_json) {
 // {"forms":[per result column],"keys":[result column indexes in key-message order],"template":[[text, code], ...]}.
 int tfgpu_emit_debezium_validate(const char* ns, const char* name, const char* schema_json, const char* transformers_json, const char* opts_json,
                                  char* describe_out, uint64_t cap, char* err_out, uint64_t err_cap) {
-    auto put = [](char* dst, uint64_t cap_, const std::string& s) { if (dst && cap_) { size_t n = s.size() < cap_ - 1 ? s.size() : cap_ - 1; std::memcpy(dst, s.data(), n); dst[n] = 0; } };
     if (!schema_json || !name || !opts_json) return TF_E_FATAL_ARG;
-    try {
+    return validated(describe_out, cap, err_out, err_cap, [&] {
         const tfplan::Plan pl = tfplan::build_plan(ns ? ns : "", name, schema_json, transformers_json ? transformers_json : "", "");
         const DbzHostTpl t = dbz_host_template(pl, opts_json);
         std::vector<size_t> order(pl.out_schema.size()); for (size_t k = 0; k < order.size(); k++) order[k] = k;
@@ -1126,12 +1203,8 @@ int tfgpu_emit_debezium_validate(const char* ns, const char* name, const char* s
             if (g) d += ",";
             d += "[" + host_json_quote_nohtml(t.text.substr((size_t)t.segs[g].text_off, (size_t)t.segs[g].text_len)) + "," + std::to_string(t.segs[g].code) + "]";
         }
-        d += "]}";
-        if (describe_out && d.size() + 1 > cap) { put(err_out, err_cap, "describe buffer too small"); return TF_E_FATAL_ARG; }
-        put(describe_out, cap, d);
-        return TF_OK;
-    } catch (const tfplan::FatalError& f) { put(err_out, err_cap, f.what()); return f.code; }
-    catch (const std::exception& x) { put(err_out, err_cap, x.what()); return TF_E_FATAL_CONFIG; }
+        return d + "]}";
+    });
 }
 
 int tfgpu_emit_debezium(tfgpu_engine* e, int plan_id, const char* opts_json, const tf_batch* in, const tf_row_meta* meta, tfgpu_result** out) {
@@ -1139,18 +1212,16 @@ int tfgpu_emit_debezium(tfgpu_engine* e, int plan_id, const char* opts_json, con
 }
 
 int tfgpu_emit_debezium_crud(tfgpu_engine* e, int plan_id, const char* opts_json, const tf_batch* in, const tf_old_keys* old, const tf_row_meta* meta, tfgpu_result** out) {
-    if (!e || !in || !out || !opts_json || plan_id < 0 || plan_id >= (int)e->plans.size()) return TF_E_FATAL_ARG;
+    PlanDev* pd = plan_arg(e, plan_id);
+    if (!pd || !in || !out || !opts_json) return TF_E_FATAL_ARG;
     *out = nullptr;
-    PlanDev& pd = *e->plans[plan_id];
-    if (in->ncols != pd.plan.in_schema.size()) return fail(e, TF_E_FATAL_ARG, "batch column count does not match the plan schema");
-    if (in->nrows >= (1ull << 31)) return fail(e, TF_E_FATAL_ARG, "batch too large (>= 2^31 rows)");
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
+        check_batch(*pd, in);
         const uint64_t n = in->nrows;
         cudaStream_t s = e->stream;
-        try { dbz_build_template(pd, opts_json); } catch (const std::runtime_error& x) { return fail(e, TF_E_FATAL_CONFIG, std::string("opts_json: ") + x.what()); }
+        try { dbz_build_template(*pd, opts_json); } catch (const std::runtime_error& x) { throw tfplan::FatalError(TF_E_FATAL_CONFIG, std::string("opts_json: ") + x.what()); }
         std::vector<tf_col> dev; const uint8_t* dev_kinds = stage_input(e, in, dev);
-        e->dbz = pd.dbz;
+        e->dbz = pd->dbz;
         const size_t o_id = 0, o_lsn = align_up(n * 4 + 16, 256), o_ct = o_lsn + align_up(n * 8 + 16, 256), o_off = o_ct + align_up(n * 8 + 16, 256), o_pre = o_off + align_up((n + 1) * 4 + 16, 256), o_heap = o_pre + align_up(n + 16, 256);
         uint64_t gt_len = 0;
         if (meta && in->mem == TF_MEM_HOST && meta->txid_offsets && meta->txid_heap) gt_len = meta->txid_offsets[n];
@@ -1171,7 +1242,7 @@ int tfgpu_emit_debezium_crud(tfgpu_engine* e, int plan_id, const char* opts_json
         // update / delete events: kinds + OldKeys (as a second set of typed columns) reach the row writer
         {
             auto ov = tfj::parse(opts_json);
-            const tfplan::Plan& pl = pd.plan; const size_t nc = pl.in_schema.size();
+            const tfplan::Plan& pl = pd->plan; const size_t nc = pl.in_schema.size();
             e->dbz.kinds = dev_kinds; e->dbz.snapshot = ov->get_bool("snapshot") ? 1 : 0; e->dbz.mysql_src = ov->get_str("source_type") == "mysql" ? 1 : 0;
             const tfj::Value* tv = ov->get("tombstones_on_delete"); e->dbz.tombstones = (tv && tv->kind == tfj::Value::Bool && !tv->b) ? 0 : 1;      // tombstones.on.delete, default true
             int npk = 0; for (const auto& c : pl.out_schema) if (c.key) npk++;
@@ -1182,10 +1253,9 @@ int tfgpu_emit_debezium_crud(tfgpu_engine* e, int plan_id, const char* opts_json
                 std::vector<tf_col> odev; stage_input(e, old->values, odev, &e->old_arena);
                 std::vector<DCol> oc(nc); std::vector<uint8_t> present(nc, 0); int np = 0;
                 for (size_t c = 0; c < nc; c++) {
-                    const tf_col& ic = odev[c]; DCol& d = oc[c]; std::memset(&d, 0, sizeof d);
+                    const tf_col& ic = odev[c];
                     if (ic.type != pl.in_schema[c].tf) return fail(e, TF_E_FATAL_ARG, "old keys: column " + std::to_string(c) + " type does not match the plan schema");
-                    d.type = ic.type; d.out_kind = OK_COPY; d.in_w = in_width(ic.type); d.out_w = d.in_w; d.str_slot = -1; d.mask_slot = -1;
-                    d.values = (const uint8_t*)ic.values; d.validity = ic.validity; d.offsets = ic.offsets; d.heap = ic.heap; d.aux = (const uint8_t*)ic.aux;
+                    DCol& d = oc[c]; d = plain_dcol(ic, ic.type); d.out_kind = OK_COPY; d.out_w = d.in_w;
                     present[c] = (old->present_cols && old->present_cols[c]) ? 1 : 0; np += present[c];
                     if (present[c] && n) { if (d.in_w && !d.values) return fail(e, TF_E_FATAL_ARG, "old keys: values pointer is NULL"); if (!d.in_w && !d.offsets) return fail(e, TF_E_FATAL_ARG, "old keys: offsets pointer is NULL"); }
                 }
@@ -1201,28 +1271,25 @@ int tfgpu_emit_debezium_crud(tfgpu_engine* e, int plan_id, const char* opts_json
                 CK(cudaStreamSynchronize(s));      // oc / present are stack vectors
             }
         }
-        run_chain(e, pd, in, dev.data(), dev_kinds, TF_WIRE_DEBEZIUM, nullptr);
+        run_chain(e, *pd, in, dev.data(), dev_kinds, TF_WIRE_DEBEZIUM, nullptr);
         auto r = std::make_unique<tfgpu_result>();
         finish_wire(e, n, TF_WIRE_DEBEZIUM, r.get());
         *out = r.release();
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
-    catch (const std::bad_alloc&) { return fail(e, TF_E_RETRY_OOM, "host allocation failed"); }
+    });
 }
 
 // Measurer middleware (synchronizer/measurer.go:38-42): Size.Values of every row and their sum, in one pass over the columns.
 int tfgpu_measure(tfgpu_engine* e, const tf_batch* in, uint64_t* per_row, uint64_t* total) {
     if (!e || !in || !total) return TF_E_FATAL_ARG;
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
         cudaStream_t s = e->stream;
         join_tail(e);                     // the work arena is reused below
         std::vector<tf_col> dev; stage_input(e, in, dev);
         const size_t nc = in->ncols; const uint64_t n = in->nrows;
         if (e->d_cols_cap < nc) { if (e->d_cols) CK(cudaFree(e->d_cols)); CK(cudaMalloc(&e->d_cols, sizeof(DCol) * (nc ? nc : 1))); e->d_cols_cap = nc; }
         std::vector<DCol> hc(nc);
-        for (size_t c = 0; c < nc; c++) { const tf_col& ic = dev[c]; DCol& d = hc[c]; std::memset(&d, 0, sizeof d); d.type = ic.type; d.in_w = in_width(ic.type); d.values = (const uint8_t*)ic.values; d.validity = ic.validity; d.offsets = ic.offsets; d.heap = ic.heap; d.aux = (const uint8_t*)ic.aux; }
+        for (size_t c = 0; c < nc; c++) hc[c] = plain_dcol(dev[c], dev[c].type);
         e->work.ensure(n * 8 + 256);
         unsigned long long* d_total = (unsigned long long*)e->work.p; uint64_t* d_rows = per_row ? (uint64_t*)(e->work.p + 64) : nullptr;
         CK(cudaMemcpyAsync(e->d_cols, hc.data(), sizeof(DCol) * nc, cudaMemcpyHostToDevice, s));
@@ -1233,9 +1300,7 @@ int tfgpu_measure(tfgpu_engine* e, const tf_batch* in, uint64_t* per_row, uint64
         if (per_row && n) CK(cudaMemcpyAsync(per_row, d_rows, n * 8, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
-    catch (const std::bad_alloc&) { return fail(e, TF_E_RETRY_OOM, "host allocation failed"); }
+    });
 }
 
 // ---------------------------------------------------------------------------------------------- CSV
@@ -1278,17 +1343,15 @@ CsvHostOpts parse_csv_opts(const char* js) {
 }  // namespace
 
 int tfgpu_parse_csv(tfgpu_engine* e, int plan_id, const char* opts_json, const uint8_t* bytes, uint64_t len, int mem, int wire_fmt, tfgpu_result** out) {
-    if (!e || !out || (!bytes && len) || plan_id < 0 || plan_id >= (int)e->plans.size()) return TF_E_FATAL_ARG;
+    PlanDev* pd = plan_arg(e, plan_id);
+    if (!pd || !out || (!bytes && len)) return TF_E_FATAL_ARG;
     *out = nullptr;
-    PlanDev& pd = *e->plans[plan_id];
-    if (len >= (1ull << 32) - 16) return fail(e, TF_E_FATAL_ARG, "csv chunk must be < 4 GiB (line positions are uint32)");
-    if (wire_fmt != 0 && !wire_known(wire_fmt)) return fail(e, TF_E_FATAL_UNSUPPORTED, "wire format not implemented");
-    if (wire_fmt != 0 && !wire_is_ser(wire_fmt) && !pd.plan.has_sink) return fail(e, TF_E_FATAL_CONFIG, "plan was built without a sink");
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
+        if (len >= (1ull << 32) - 16) throw tfplan::FatalError(TF_E_FATAL_ARG, "csv chunk must be < 4 GiB (line positions are uint32)");
+        check_wire(*pd, wire_fmt, true);
         cudaStream_t s = e->stream;
         CsvHostOpts ho = parse_csv_opts(opts_json);
-        const tfplan::Plan& pl = pd.plan; const size_t nc = pl.in_schema.size();
+        const tfplan::Plan& pl = pd->plan; const size_t nc = pl.in_schema.size();
         // text into HBM
         const uint8_t* d_text = bytes;
         if (mem == TF_MEM_HOST) { e->csv_text.ensure(len + 64); if (len) CK(cudaMemcpyAsync(e->csv_text.p, bytes, len, cudaMemcpyHostToDevice, s)); d_text = e->csv_text.p; }
@@ -1308,19 +1371,19 @@ int tfgpu_parse_csv(tfgpu_engine* e, int plan_id, const char* opts_json, const u
         const uint64_t skip = ho.skip < nlines ? ho.skip : nlines;
         const uint64_t nrows = nlines - skip;
         // staging layout
-        std::vector<CsvColDev> hc(nc); std::vector<int16_t> next_same(nc, -1); int nfields = 0, nslots = 0, nany = 0;
+        std::vector<CsvColDev> hc(nc); std::vector<int16_t> next_same(nc, -1); int nfields = 0, nslots = 0;
         for (size_t c = 0; c < nc; c++) {
             const tfplan::ColSchema& cs = pl.in_schema[c]; CsvColDev& d = hc[c]; std::memset(&d, 0, sizeof d);
             d.tf = cs.tf; d.w = in_width(cs.tf); d.slot = -1;
             d.path = cs.path.empty() ? (int)c : atoi(cs.path.c_str());        // reader_csv.go:286 strconv.Atoi(col.Path)
             if (!cs.path.empty() && cs.path.find_first_not_of("-0123456789") != std::string::npos) throw tfplan::FatalError(TF_E_FATAL_CONFIG, "csv: column path '" + cs.path + "' is not an index");
             if (d.path >= 0 && d.path + 1 > nfields) nfields = d.path + 1;
-            if (!d.w) { d.slot = nslots++; if (cs.tf == TF_ANY) nany++; }
+            if (!d.w) d.slot = nslots++;
         }
         if (nfields > 32000) throw tfplan::FatalError(TF_E_FATAL_UNSUPPORTED, "csv: too many fields");
         std::vector<int16_t> field_col(nfields ? nfields : 1, -1);
         for (int c = (int)nc - 1; c >= 0; c--) if (hc[c].path >= 0) { next_same[c] = field_col[hc[c].path]; field_col[hc[c].path] = (int16_t)c; }
-        size_t sb = 0; auto need = [&](size_t b) { size_t at = sb; sb += align_up(b ? b : 1, 256); return at; };
+        ArenaLayout need;
         const size_t o_line = need((nlines + 1) * 4), o_err = need(nrows), o_cols = need(nc * sizeof(CsvColDev)), o_fc = need(field_col.size() * 2), o_ns = need(nc * 2),
                      o_blob = need(ho.blob.size()), o_ss = need((size_t)nslots * nrows * 4), o_sl = need((size_t)nslots * nrows * 4),
                      o_off = need((size_t)nslots * (nrows + 1) * 4), o_tot = need((size_t)nslots * 8 + 8), o_base = need((size_t)nslots * 8 + 8);
@@ -1330,8 +1393,7 @@ int tfgpu_parse_csv(tfgpu_engine* e, int plan_id, const char* opts_json, const u
             const int tf = hc[c].tf;
             o_aux[c] = (tf == TF_DATE || tf == TF_DATETIME || tf == TF_TIMESTAMP) ? need(4 * nrows) : (tf == TF_ANY ? need(nrows) : 0);
         }
-        const size_t o_heap = need(len + 2 * nrows * (size_t)(nany ? nany : 0) + 64);
-        e->csv_stage.ensure(sb + 256);
+        e->csv_stage.ensure(need.total + 256);
         uint8_t* B = e->csv_stage.p;
         for (size_t c = 0; c < nc; c++) {
             if (hc[c].w) hc[c].values = B + o_val[c];
@@ -1343,43 +1405,26 @@ int tfgpu_parse_csv(tfgpu_engine* e, int plan_id, const char* opts_json, const u
         CK(cudaMemcpyAsync(B + o_fc, field_col.data(), field_col.size() * 2, cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(B + o_ns, next_same.data(), nc * 2, cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(B + o_blob, ho.blob.data(), ho.blob.size(), cudaMemcpyHostToDevice, s));
-        std::vector<uint64_t> col_total(nslots ? nslots : 1, 0), col_base(nslots ? nslots : 1, 0);
+        VarHeaps heaps(nslots);
         if (nlines) { e->prof_begin("k_csv_line_index", s); launch_k_csv_line_index(nblk, 256, 0, s, d_text, len, blk_off, (uint32_t*)(B + o_line), nullptr); e->prof_end(s); }
         if (nrows) {
             CsvArgs ca{d_text, len, (const uint32_t*)(B + o_line), nlines, skip, ho.cfg, B + o_blob, (const CsvColDev*)(B + o_cols), (int)nc,
                        (const int16_t*)(B + o_fc), nfields, (const int16_t*)(B + o_ns), (uint32_t*)(B + o_ss), (uint32_t*)(B + o_sl), B + o_err};
             e->prof_begin("k_csv_pass1", s); launch_k_csv_pass1((uint32_t)std::min<uint64_t>((nrows + CSV_TILE_ROWS - 1) / CSV_TILE_ROWS, (uint64_t)e->sm_count * 16), 32 * CSV_WARPS, 0, s, ca); e->prof_end(s);
             if (nslots) {
-                launch_offsets(e, (const uint32_t*)(B + o_sl), nrows, (uint32_t)nslots, (uint32_t*)(B + o_off), (uint64_t*)(B + o_tot), s);
-                CK(cudaMemcpyAsync(col_total.data(), B + o_tot, (size_t)nslots * 8, cudaMemcpyDeviceToHost, s)); CK(cudaStreamSynchronize(s));
-                uint64_t run = 0; for (int k = 0; k < nslots; k++) { col_base[k] = run; run += col_total[k]; }
-                CK(cudaMemcpyAsync(B + o_base, col_base.data(), (size_t)nslots * 8, cudaMemcpyHostToDevice, s));
-                CsvCopyArgs cp{d_text, (const uint32_t*)(B + o_ss), (const uint32_t*)(B + o_sl), (const uint32_t*)(B + o_off), B + o_heap, (const uint64_t*)(B + o_base), nrows};
+                place_heaps(e, heaps, (const uint32_t*)(B + o_sl), nrows, nslots, (uint32_t*)(B + o_off), (uint64_t*)(B + o_tot), (uint64_t*)(B + o_base), "csv chunk");
+                CsvCopyArgs cp{d_text, (const uint32_t*)(B + o_ss), (const uint32_t*)(B + o_sl), (const uint32_t*)(B + o_off), heaps.heap, (const uint64_t*)(B + o_base), nrows};
                 e->prof_begin("k_csv_pass2", s); launch_k_csv_pass2(dim3((uint32_t)((nrows + 255) / 256), nslots), 256, 0, s, cp); e->prof_end(s);
             }
         }
-        // the staged batch, device resident
-        std::vector<tf_col> dev(nc);
-        for (size_t c = 0; c < nc; c++) {
-            tf_col& d = dev[c]; std::memset(&d, 0, sizeof d); d.type = hc[c].tf;
-            if (hc[c].w) { d.values = hc[c].values; d.aux = hc[c].aux32; }
-            else { d.offsets = (const uint32_t*)(B + o_off) + (size_t)hc[c].slot * (nrows + 1); d.heap = B + o_heap + col_base[hc[c].slot]; d.heap_len = col_total[hc[c].slot]; d.aux = hc[c].aux8; }
-        }
-        tf_batch staged; staged.nrows = nrows; staged.ncols = (uint32_t)nc; staged.mem = TF_MEM_DEVICE; staged.cols = dev.data(); staged.kinds = nullptr;
-        const int saved_prof = e->prof_n;
-        run_chain(e, pd, &staged, dev.data(), nullptr, wire_fmt == 0 ? TF_WIRE_COLUMNAR_INTERNAL : wire_fmt, nrows ? B + o_err : nullptr);
-        (void)saved_prof;
-        auto r = std::make_unique<tfgpu_result>();
-        if (wire_fmt == 0) finish_columnar(e, pd, nrows, r.get()); else finish_wire(e, nrows, wire_fmt, r.get());
+        std::vector<tf_col> dev;
+        auto r = chain_parsed(e, *pd, parsed_batch(hc, nrows, (const uint32_t*)(B + o_off), heaps, dev), nullptr, nrows ? B + o_err : nullptr, wire_fmt);
         uint32_t last_end = 0;
         if (nlines) { CK(cudaMemcpyAsync(&last_end, (uint32_t*)(B + o_line) + (nlines - 1), 4, cudaMemcpyDeviceToHost, s)); CK(cudaStreamSynchronize(s)); }
         r->consumed = last_end;
         *out = r.release();
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
-    catch (const std::bad_alloc&) { return fail(e, TF_E_RETRY_OOM, "host allocation failed"); }
-    catch (const std::exception& x) { return fail(e, TF_E_FATAL_CONFIG, x.what()); }
+    });
 }
 
 // ---------------------------------------------------------------------------------------------- JSON lines
@@ -1387,18 +1432,15 @@ int tfgpu_parse_csv(tfgpu_engine* e, int plan_id, const char* opts_json, const u
 // transformer chain and the sink encode: message bytes in, Transformed rows or wire bytes out.
 int tfgpu_parse_json(tfgpu_engine* e, int plan_id, const char* opts_json, const uint8_t* bytes, uint64_t len, int mem,
                      const tf_msg* msgs, uint32_t n_msgs, int wire_fmt, tfgpu_result** out) {
-    if (!e || !out || (!bytes && len) || (!msgs && n_msgs) || plan_id < 0 || plan_id >= (int)e->plans.size()) return TF_E_FATAL_ARG;
+    PlanDev* pd = plan_arg(e, plan_id);
+    if (!pd || !out || (!bytes && len) || (!msgs && n_msgs)) return TF_E_FATAL_ARG;
     *out = nullptr;
-    PlanDev& pd = *e->plans[plan_id];
-    if (len >= (1ull << 32) - 16) return fail(e, TF_E_FATAL_ARG, "json batch must be < 4 GiB (line positions are uint32)");
-    if (wire_fmt != 0 && !wire_known(wire_fmt)) return fail(e, TF_E_FATAL_UNSUPPORTED, "wire format not implemented");
-    if (wire_fmt != 0 && !wire_is_ser(wire_fmt) && !pd.plan.has_sink) return fail(e, TF_E_FATAL_CONFIG, "plan was built without a sink");
-    { uint64_t prev = 0; for (uint32_t m = 0; m < n_msgs; m++) { if (msgs[m].end < prev || msgs[m].end > len) return fail(e, TF_E_FATAL_ARG, "message ends must be non-decreasing and inside the buffer"); prev = msgs[m].end; }
-      if ((n_msgs ? msgs[n_msgs - 1].end : 0) != len) return fail(e, TF_E_FATAL_ARG, "the messages must cover the whole buffer"); }
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
+        if (len >= (1ull << 32) - 16) throw tfplan::FatalError(TF_E_FATAL_ARG, "json batch must be < 4 GiB (line positions are uint32)");
+        check_wire(*pd, wire_fmt, true);
+        check_msg_ends(len, n_msgs, [&](uint32_t m) { return msgs[m].end; });
         cudaStream_t s = e->stream;
-        const tfplan::Plan& pl = pd.plan; const size_t nc = pl.in_schema.size();
+        const tfplan::Plan& pl = pd->plan; const size_t nc = pl.in_schema.size();
         // ---- options (AuxParserOpts, generic_parser.go:41-84)
         bool add_rest = false, add_dedupe = false, nka = false, use_numbers = false, b64 = false; std::string partition;
         if (opts_json && *opts_json) {
@@ -1441,10 +1483,10 @@ int tfgpu_parse_json(tfgpu_engine* e, int plan_id, const char* opts_json, const 
         std::vector<uint64_t> h_end(n_msgs ? n_msgs : 1), h_off(n_msgs ? n_msgs : 1); std::vector<int64_t> h_ws(n_msgs ? n_msgs : 1); std::vector<uint32_t> h_wn(n_msgs ? n_msgs : 1);
         for (uint32_t m = 0; m < n_msgs; m++) { h_end[m] = msgs[m].end; h_off[m] = msgs[m].offset; h_ws[m] = msgs[m].write_sec; h_wn[m] = msgs[m].write_nsec; }
         {
-            size_t wb = 0; auto need = [&](size_t b) { size_t at = wb; wb += align_up(b ? b : 1, 256); return at; };
+            ArenaLayout need;
             const size_t w_cnt = need(((size_t)nblk + 64) * 4), w_off = need(((size_t)nblk + 64) * 4), w_bits = need(bits_words * 4),
                          w_end = need((size_t)n_msgs * 8), w_moff = need((size_t)n_msgs * 8), w_ws = need((size_t)n_msgs * 8), w_wn = need((size_t)n_msgs * 4), w_r0 = need((size_t)n_msgs * 4);
-            e->json_msgs.ensure(wb + 256);                       // message table + line-count scratch live here until the text heap is sized
+            e->json_msgs.ensure(need.total + 256);                // message table + line-count scratch live here until the text heap is sized
             uint8_t* W = e->json_msgs.p;
             uint32_t* blk_cnt = (uint32_t*)(W + w_cnt); uint32_t* blk_off = (uint32_t*)(W + w_off); uint32_t* endbits = (uint32_t*)(W + w_bits);
             uint64_t nlines = 0;
@@ -1462,7 +1504,7 @@ int tfgpu_parse_json(tfgpu_engine* e, int plan_id, const char* opts_json, const 
             }
             const uint64_t nrows = nlines;
             // ---- staging layout (csv_stage arena)
-            size_t sb = 0; auto sneed = [&](size_t b) { size_t at = sb; sb += align_up(b ? b : 1, 256); return at; };
+            ArenaLayout sneed;
             const uint32_t nlb = (uint32_t)((nlines + 127) / 128);
             const size_t o_line = sneed((nlines + 1) * 4), o_rank = sneed((nlines + 2) * 4), o_lcnt = sneed(((size_t)nlb + 64) * 4), o_loff = sneed(((size_t)nlb + 64) * 4),
                          o_err = sneed(nrows), o_ecol = sneed(nrows), o_cols = sneed(nc * sizeof(JsnColDev)), o_names = sneed(names.size()),
@@ -1475,7 +1517,7 @@ int tfgpu_parse_json(tfgpu_engine* e, int plan_id, const char* opts_json, const 
                 o_aux[c] = (tf == TF_DATE || tf == TF_DATETIME || tf == TF_TIMESTAMP) ? sneed(4 * nrows) : (tf == TF_ANY ? sneed(nrows) : 0);
                 o_vld[c] = sneed((nrows / 32 + 2) * 4);
             }
-            e->csv_stage.ensure(sb + 256);
+            e->csv_stage.ensure(sneed.total + 256);
             uint8_t* B = e->csv_stage.p;
             for (size_t c = 0; c < nc; c++) {
                 if (hc[c].w) hc[c].values = B + o_val[c];
@@ -1484,9 +1526,8 @@ int tfgpu_parse_json(tfgpu_engine* e, int plan_id, const char* opts_json, const 
                 if (tf == TF_ANY) hc[c].aux8 = B + o_aux[c];
                 hc[c].validity = (uint32_t*)(B + o_vld[c]);
             }
-            std::vector<uint64_t> col_total(nslots ? nslots : 1, 0), col_base(nslots ? nslots : 1, 0);
+            VarHeaps heaps(nslots);
             uint32_t n_nonempty = 0;
-            const uint8_t* heap = nullptr;
             if (nrows) {
                 CK(cudaMemcpyAsync(B + o_cols, hc.data(), nc * sizeof(JsnColDev), cudaMemcpyHostToDevice, s));
                 CK(cudaMemcpyAsync(B + o_names, names.data(), names.size(), cudaMemcpyHostToDevice, s));
@@ -1508,28 +1549,13 @@ int tfgpu_parse_json(tfgpu_engine* e, int plan_id, const char* opts_json, const 
                 e->prof_begin("k_json_pass1", s); launch_k_json_pass1(nlb, 128, JSN_STAGE, s, ja); e->prof_end(s);
                 CK(cudaMemcpyAsync(&n_nonempty, (uint32_t*)(B + o_rank) + nlines, 4, cudaMemcpyDeviceToHost, s));
                 if (nslots) {
-                    launch_offsets(e, (const uint32_t*)(B + o_len), nrows, (uint32_t)nslots, (uint32_t*)(B + o_off), (uint64_t*)(B + o_tot), s);
-                    CK(cudaMemcpyAsync(col_total.data(), B + o_tot, (size_t)nslots * 8, cudaMemcpyDeviceToHost, s)); CK(cudaStreamSynchronize(s));
-                    uint64_t run = 0; for (int k = 0; k < nslots; k++) { col_base[k] = run; run += align_up(col_total[k], 16); }
-                    if (run >= (1ull << 32)) throw tfplan::FatalError(TF_E_FATAL_ARG, "json batch: a text column exceeds 4 GiB");
-                    e->in_arena.ensure(run + 256);               // text heaps (the staged batch is device resident, in_arena is free)
-                    heap = e->in_arena.p;
-                    CK(cudaMemcpyAsync(B + o_base, col_base.data(), (size_t)nslots * 8, cudaMemcpyHostToDevice, s));
-                    JsnWriteArgs wa{ja, (const uint32_t*)(B + o_off), e->in_arena.p, (const uint64_t*)(B + o_base)};
+                    place_heaps(e, heaps, (const uint32_t*)(B + o_len), nrows, nslots, (uint32_t*)(B + o_off), (uint64_t*)(B + o_tot), (uint64_t*)(B + o_base), "json batch");
+                    JsnWriteArgs wa{ja, (const uint32_t*)(B + o_off), heaps.heap, (const uint64_t*)(B + o_base)};
                     e->prof_begin("k_json_pass2", s); launch_k_json_pass2(nlb, 128, JSN_STAGE, s, wa); e->prof_end(s);
                 } else CK(cudaStreamSynchronize(s));
             }
-            // ---- the staged batch, device resident
-            std::vector<tf_col> dev(nc);
-            for (size_t c = 0; c < nc; c++) {
-                tf_col& d = dev[c]; std::memset(&d, 0, sizeof d); d.type = hc[c].tf; d.validity = (const uint8_t*)hc[c].validity;
-                if (hc[c].w) { d.values = hc[c].values; d.aux = hc[c].aux32; }
-                else { d.offsets = (const uint32_t*)(B + o_off) + (size_t)hc[c].slot * (nrows + 1); d.heap = heap ? heap + col_base[hc[c].slot] : nullptr; d.heap_len = col_total[hc[c].slot]; d.aux = hc[c].aux8; }
-            }
-            tf_batch staged; staged.nrows = nrows; staged.ncols = (uint32_t)nc; staged.mem = TF_MEM_DEVICE; staged.cols = dev.data(); staged.kinds = nullptr;
-            run_chain(e, pd, &staged, dev.data(), nullptr, wire_fmt == 0 ? TF_WIRE_COLUMNAR_INTERNAL : wire_fmt, nrows ? B + o_err : nullptr);
-            auto r = std::make_unique<tfgpu_result>();
-            if (wire_fmt == 0) finish_columnar(e, pd, nrows, r.get()); else finish_wire(e, nrows, wire_fmt, r.get());
+            std::vector<tf_col> dev;
+            auto r = chain_parsed(e, *pd, parsed_batch(hc, nrows, (const uint32_t*)(B + o_off), heaps, dev), nullptr, nrows ? B + o_err : nullptr, wire_fmt);
             // row errors: row = index among the NON-EMPTY lines (empty lines are not lines to the reference, :528-530), term = column
             if (!r->errs.empty()) {
                 std::vector<uint8_t> ecol(nrows); CK(cudaMemcpyAsync(ecol.data(), B + o_ecol, nrows, cudaMemcpyDeviceToHost, s)); CK(cudaStreamSynchronize(s));
@@ -1542,10 +1568,7 @@ int tfgpu_parse_json(tfgpu_engine* e, int plan_id, const char* opts_json, const 
             *out = r.release();
         }
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
-    catch (const std::bad_alloc&) { return fail(e, TF_E_RETRY_OOM, "host allocation failed"); }
-    catch (const std::exception& x) { return fail(e, TF_E_FATAL_CONFIG, x.what()); }
+    });
 }
 
 // ---------------------------------------------------------------------------------------------- Debezium
@@ -1577,18 +1600,21 @@ std::vector<DbzHostField> dbz_fields(const tfj::Value& schema, const char* which
     }
     return out;
 }
+// The table fields of an envelope schema: those of its `after` struct, which the `before` struct must repeat.
+std::vector<DbzHostField> dbz_table_fields(const tfj::Value& schema) {
+    const std::vector<DbzHostField> fs = dbz_fields(schema, "after"), fb = dbz_fields(schema, "before");
+    auto same = [](const DbzHostField& a, const DbzHostField& b) { return a.name == b.name && a.recv == b.recv && a.scale == b.scale; };
+    if (!std::equal(fs.begin(), fs.end(), fb.begin(), fb.end(), same)) throw tfplan::FatalError(TF_E_FATAL_UNSUPPORTED, "debezium: 'before' and 'after' structs differ");
+    return fs;
+}
 }  // namespace
 
 // Host-only: the table schema and receivers tfgpu_parse_debezium derives from a Kafka Connect envelope schema (no GPU needed):
 // [{"name","type","key","recv","scale"}, ...] in the order of the `after` struct, or the error the call would return.
 int tfgpu_debezium_schema_validate(const char* schema_text, char* describe_out, uint64_t cap, char* err_out, uint64_t err_cap) {
-    auto put = [](char* dst, uint64_t cap_, const std::string& s) { if (dst && cap_) { size_t n = s.size() < cap_ - 1 ? s.size() : cap_ - 1; std::memcpy(dst, s.data(), n); dst[n] = 0; } };
     if (!schema_text) return TF_E_FATAL_ARG;
-    try {
-        auto sv = tfj::parse(schema_text);
-        const std::vector<DbzHostField> fs = dbz_fields(*sv, "after"), fb = dbz_fields(*sv, "before");
-        if (fs.size() != fb.size()) throw tfplan::FatalError(TF_E_FATAL_UNSUPPORTED, "debezium: 'before' and 'after' structs differ");
-        for (size_t i = 0; i < fs.size(); i++) if (fs[i].name != fb[i].name || fs[i].recv != fb[i].recv || fs[i].scale != fb[i].scale) throw tfplan::FatalError(TF_E_FATAL_UNSUPPORTED, "debezium: 'before' and 'after' structs differ");
+    return validated(describe_out, cap, err_out, err_cap, [&] {
+        const std::vector<DbzHostField> fs = dbz_table_fields(*tfj::parse(schema_text));
         static const char* yt[] = {"", "int8", "int16", "int32", "int64", "uint8", "uint16", "uint32", "uint64", "float", "double", "boolean", "string", "utf8", "any", "date", "datetime", "timestamp", "interval"};
         std::string d = "[";
         for (size_t i = 0; i < fs.size(); i++) {
@@ -1596,37 +1622,27 @@ int tfgpu_debezium_schema_validate(const char* schema_text, char* describe_out, 
             d += "{\"name\":" + host_json_quote_nohtml(fs[i].name) + ",\"type\":\"" + yt[fs[i].tf] + "\",\"key\":" + (fs[i].key ? "true" : "false") +
                  ",\"recv\":" + std::to_string(fs[i].recv) + ",\"scale\":" + std::to_string(fs[i].scale) + "}";
         }
-        d += "]";
-        if (describe_out && d.size() + 1 > cap) { put(err_out, err_cap, "describe buffer too small"); return TF_E_FATAL_ARG; }
-        put(describe_out, cap, d);
-        return TF_OK;
-    } catch (const tfplan::FatalError& f) { put(err_out, err_cap, f.what()); return f.code; }
-    catch (const std::exception& x) { put(err_out, err_cap, x.what()); return TF_E_FATAL_CONFIG; }
+        return d + "]";
+    });
 }
 
 int tfgpu_parse_debezium(tfgpu_engine* e, int plan_id, const char* opts_json, const uint8_t* bytes, uint64_t len, int mem,
                          const uint64_t* msg_ends, uint32_t n_msgs, int wire_fmt, tfgpu_result** out) {
-    if (!e || !out || !opts_json || (!bytes && len) || (!msg_ends && n_msgs) || plan_id < 0 || plan_id >= (int)e->plans.size()) return TF_E_FATAL_ARG;
+    PlanDev* pd = plan_arg(e, plan_id);
+    if (!pd || !out || !opts_json || (!bytes && len) || (!msg_ends && n_msgs)) return TF_E_FATAL_ARG;
     *out = nullptr;
-    PlanDev& pd = *e->plans[plan_id];
-    if (len >= (1ull << 32) - 16) return fail(e, TF_E_FATAL_ARG, "debezium batch must be < 4 GiB");
-    if (wire_fmt != 0 && !wire_known(wire_fmt)) return fail(e, TF_E_FATAL_UNSUPPORTED, "wire format not implemented");
-    if (wire_fmt != 0 && !wire_is_ser(wire_fmt) && !pd.plan.has_sink) return fail(e, TF_E_FATAL_CONFIG, "plan was built without a sink");
-    { uint64_t prev = 0; for (uint32_t m = 0; m < n_msgs; m++) { if (msg_ends[m] < prev || msg_ends[m] > len) return fail(e, TF_E_FATAL_ARG, "message ends must be non-decreasing and inside the buffer"); prev = msg_ends[m]; }
-      if ((n_msgs ? msg_ends[n_msgs - 1] : 0) != len) return fail(e, TF_E_FATAL_ARG, "the messages must cover the whole buffer"); }
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
+        if (len >= (1ull << 32) - 16) throw tfplan::FatalError(TF_E_FATAL_ARG, "debezium batch must be < 4 GiB");
+        check_wire(*pd, wire_fmt, true);
+        check_msg_ends(len, n_msgs, [&](uint32_t m) { return msg_ends[m]; });
         cudaStream_t s = e->stream;
-        const tfplan::Plan& pl = pd.plan; const size_t nc = pl.in_schema.size();
+        const tfplan::Plan& pl = pd->plan; const size_t nc = pl.in_schema.size();
         auto ov = tfj::parse(opts_json);
         const std::string schema_text = ov->get_str("schema_text");
         const bool use_sr = ov->get_bool("schema_registry"), check_table = ov->get_bool("check_table");
         const uint32_t schema_id = (uint32_t)ov->get_num("schema_id", 0);
         if (schema_text.empty()) throw tfplan::FatalError(TF_E_FATAL_CONFIG, "debezium: opts.schema_text (the Kafka Connect schema this plan was built for) is required");
-        auto sv = tfj::parse(schema_text.c_str());
-        const std::vector<DbzHostField> fs = dbz_fields(*sv, "after"), fb = dbz_fields(*sv, "before");
-        if (fs.size() != fb.size()) throw tfplan::FatalError(TF_E_FATAL_UNSUPPORTED, "debezium: 'before' and 'after' structs differ");
-        for (size_t i = 0; i < fs.size(); i++) if (fs[i].name != fb[i].name || fs[i].recv != fb[i].recv || fs[i].scale != fb[i].scale) throw tfplan::FatalError(TF_E_FATAL_UNSUPPORTED, "debezium: 'before' and 'after' structs differ");
+        const std::vector<DbzHostField> fs = dbz_table_fields(*tfj::parse(schema_text.c_str()));
         if (fs.size() != nc || nc > JSN_MAX_COLS) throw tfplan::FatalError(TF_E_FATAL_CONFIG, "debezium: the plan schema must be the table schema of the 'after' struct (at most 128 columns)");
         std::vector<DbzColDev> hc(nc); std::vector<uint8_t> names; int nslots = 0;
         for (size_t c = 0; c < nc; c++) {
@@ -1643,17 +1659,16 @@ int tfgpu_parse_debezium(tfgpu_engine* e, int plan_id, const char* opts_json, co
         const uint8_t* d_text = bytes;
         if (mem == TF_MEM_HOST) { e->csv_text.ensure(len + 64); if (len) CK(cudaMemcpyAsync(e->csv_text.p, bytes, len, cudaMemcpyHostToDevice, s)); d_text = e->csv_text.p; }
         const uint64_t n = n_msgs;
-        size_t sb = 0; auto need = [&](size_t b) { size_t at = sb; sb += align_up(b ? b : 1, 256); return at; };
+        ArenaLayout need;
         const size_t o_end = need(n * 8), o_err = need(n), o_ecol = need(n), o_cols = need(nc * sizeof(DbzColDev)), o_names = need(names.size()),
                      o_ss = need(nc * n * 4), o_sl = need(nc * n * 4), o_len = need((size_t)nslots * n * 4), o_off = need((size_t)nslots * (n + 1) * 4),
                      o_tot = need((size_t)nslots * 8 + 8), o_base = need((size_t)nslots * 8 + 8), o_kind = need(n), o_tx = need(n * 4), o_lsn = need(n * 8), o_ct = need(n * 8);
         std::vector<size_t> o_val(nc), o_vld(nc);
         for (size_t c = 0; c < nc; c++) { o_val[c] = hc[c].w ? need((size_t)hc[c].w * n) : 0; o_vld[c] = need((n / 32 + 2) * 4); }
-        e->csv_stage.ensure(sb + 256);
+        e->csv_stage.ensure(need.total + 256);
         uint8_t* B = e->csv_stage.p;
         for (size_t c = 0; c < nc; c++) { if (hc[c].w) hc[c].values = B + o_val[c]; hc[c].validity = (uint32_t*)(B + o_vld[c]); }
-        std::vector<uint64_t> col_total(nslots ? nslots : 1, 0), col_base(nslots ? nslots : 1, 0);
-        const uint8_t* heap = nullptr;
+        VarHeaps heaps(nslots);
         e->prof_n = 0;
         if (n) {
             CK(cudaMemcpyAsync(B + o_end, msg_ends, n * 8, cudaMemcpyHostToDevice, s));
@@ -1669,27 +1684,14 @@ int tfgpu_parse_debezium(tfgpu_engine* e, int plan_id, const char* opts_json, co
             const uint32_t nb = (uint32_t)((n + 127) / 128);
             e->prof_begin("k_dbz_pass1", s); launch_k_dbz_pass1(nb, 128, DBZ_STAGE, s, da); e->prof_end(s);
             if (nslots) {
-                launch_offsets(e, (const uint32_t*)(B + o_len), n, (uint32_t)nslots, (uint32_t*)(B + o_off), (uint64_t*)(B + o_tot), s);
-                CK(cudaMemcpyAsync(col_total.data(), B + o_tot, (size_t)nslots * 8, cudaMemcpyDeviceToHost, s)); CK(cudaStreamSynchronize(s));
-                uint64_t run = 0; for (int k = 0; k < nslots; k++) { col_base[k] = run; run += align_up(col_total[k], 16); }
-                if (run >= (1ull << 32)) throw tfplan::FatalError(TF_E_FATAL_ARG, "debezium batch: a text column exceeds 4 GiB");
-                e->in_arena.ensure(run + 256); heap = e->in_arena.p;
-                CK(cudaMemcpyAsync(B + o_base, col_base.data(), (size_t)nslots * 8, cudaMemcpyHostToDevice, s));
-                DbzWriteArgs wa{da, (const uint32_t*)(B + o_off), e->in_arena.p, (const uint64_t*)(B + o_base)};
+                place_heaps(e, heaps, (const uint32_t*)(B + o_len), n, nslots, (uint32_t*)(B + o_off), (uint64_t*)(B + o_tot), (uint64_t*)(B + o_base), "debezium batch");
+                DbzWriteArgs wa{da, (const uint32_t*)(B + o_off), heaps.heap, (const uint64_t*)(B + o_base)};
                 e->prof_begin("k_dbz_pass2", s); launch_k_dbz_pass2(nb, 128, 0, s, wa); e->prof_end(s);
             }
             CK(cudaGetLastError());
         }
-        std::vector<tf_col> dev(nc);
-        for (size_t c = 0; c < nc; c++) {
-            tf_col& d = dev[c]; std::memset(&d, 0, sizeof d); d.type = hc[c].tf; d.validity = (const uint8_t*)hc[c].validity;
-            if (hc[c].w) d.values = hc[c].values;
-            else { d.offsets = (const uint32_t*)(B + o_off) + (size_t)hc[c].slot * (n + 1); d.heap = heap ? heap + col_base[hc[c].slot] : nullptr; d.heap_len = col_total[hc[c].slot]; }
-        }
-        tf_batch staged; staged.nrows = n; staged.ncols = (uint32_t)nc; staged.mem = TF_MEM_DEVICE; staged.cols = dev.data(); staged.kinds = nullptr;
-        run_chain(e, pd, &staged, dev.data(), n ? B + o_kind : nullptr, wire_fmt == 0 ? TF_WIRE_COLUMNAR_INTERNAL : wire_fmt, n ? B + o_err : nullptr);
-        auto r = std::make_unique<tfgpu_result>();
-        if (wire_fmt == 0) finish_columnar(e, pd, n, r.get()); else finish_wire(e, n, wire_fmt, r.get());
+        std::vector<tf_col> dev;
+        auto r = chain_parsed(e, *pd, parsed_batch(hc, n, (const uint32_t*)(B + o_off), heaps, dev), n ? B + o_kind : nullptr, n ? B + o_err : nullptr, wire_fmt);
         if (n) {
             if (!r->errs.empty()) { std::vector<uint8_t> ecol(n); CK(cudaMemcpyAsync(ecol.data(), B + o_ecol, n, cudaMemcpyDeviceToHost, s)); CK(cudaStreamSynchronize(s)); for (auto& x : r->errs) if (x.term == 0xff) x.term = ecol[x.row]; }
             r->meta_kinds.resize(n); r->meta_tx.resize(n); r->meta_lsn.resize(n); r->meta_ct.resize(n); r->selection.resize(r->rows_out);
@@ -1701,22 +1703,18 @@ int tfgpu_parse_debezium(tfgpu_engine* e, int plan_id, const char* opts_json, co
         r->consumed = len;
         *out = r.release();
         return TF_OK;
-    } catch (const tfplan::FatalError& f) { return fail(e, f.code, f.what()); }
-    catch (const CudaError& c) { return cuda_fail(e, c); }
-    catch (const std::bad_alloc&) { return fail(e, TF_E_RETRY_OOM, "host allocation failed"); }
-    catch (const std::exception& x) { return fail(e, TF_E_FATAL_CONFIG, x.what()); }
+    });
 }
 
 // debug / profiling aid: cycles thread 0 of every k_lz4_frames CTA spent per phase since enabling (stage, match, parse, scan, emit)
 int tfgpu_debug_lz4_phases(tfgpu_engine* e, int enable, uint64_t out[8]) {
     if (!e) return TF_E_FATAL_ARG;
-    try {
-        CK(cudaSetDevice(e->device));
+    return guarded(e, [&] {
         if (enable && !e->lz_phases) { CK(cudaMalloc(&e->lz_phases, 64)); CK(cudaMemset(e->lz_phases, 0, 64)); }
         if (out && e->lz_phases) { CK(cudaStreamSynchronize(e->stream)); CK(cudaMemcpy(out, e->lz_phases, 64, cudaMemcpyDeviceToHost)); CK(cudaMemset(e->lz_phases, 0, 64)); }
         if (!enable && e->lz_phases) { CK(cudaFree(e->lz_phases)); e->lz_phases = nullptr; }
         return TF_OK;
-    } catch (const CudaError& c) { return cuda_fail(e, c); }
+    });
 }
 
 const uint32_t* tfgpu_result_dbz_msg_sizes(const tfgpu_result* r) { return (r && !r->msg_sizes.empty()) ? r->msg_sizes.data() : nullptr; }
